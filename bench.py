@@ -170,6 +170,25 @@ def bench_config(wl_name, frames_per_gpu, world, la, flush, surfels_at_end=None,
     return cfg
 
 
+def dump_outputs(ctx, out_dir, limit=64 << 20):
+    """Writes what a caller of processFrame receives after the last timed frame to out_dir/<name>.npy: the camera pose, the
+    model views predicted for the next frame (vertex, normal, colour), the surfel count and the surfel map. Above `limit` bytes in
+    all, the map is a fixed seeded sample of its rows, kept in map order (the map's compaction preserves order). Every value is
+    finite: the undefined normal of a surfel at a depth edge (NaN in the map) is written as the zero vector, which no unit normal
+    can be."""
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"pose": ctx.get_pose(), "surfel_count": np.array([ctx.map_count()], np.float64)}
+    for name in ("VERTEX", "NORMAL", "IMAGE"):
+        out[f"model_{name.lower()}"] = ctx.download(name).astype(np.float32)
+    surfels = ctx.map_download()
+    rows = max(0, limit - sum(a.nbytes for a in out.values())) // (12 * 4)
+    if len(surfels) > rows:
+        surfels = surfels[np.sort(np.random.default_rng(0).choice(len(surfels), rows, replace=False))]
+    out["surfels"] = surfels
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.where(np.isfinite(a), a, 0).astype(a.dtype))
+
+
 def populate_map(ctx, K, n_resident, seed, rgb0, depth0):
     """Frame 0 through the public call (tick 1 builds the map from the frame), then replaces the map by ~n_resident stable surfels
     tiling the room (the pose after frame 0 is the identity = the world frame of the sequence) and re-renders the model view."""
@@ -288,6 +307,8 @@ def run_ours(args, rank, world, dist):
     dev_ms = float(sum(frame_ms))
     n_surfels = ctx.map_count()
     pose = ctx.get_pose()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(ctx, args.dump_outputs)
 
     # ---------------- roofline: ICP reduction at level 0, cold L2 ----------------
     roof = icp_roofline(ctx, stream, flush, K, rgb, depth, local)
@@ -731,6 +752,7 @@ def main():
     ap.add_argument("--no-lookahead", action="store_true", help="process each frame without staging its successor on the side stream")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--quick", action="store_true", help="headline numbers only: no 1280x960 / large-map / no-look-ahead extras")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed frames, write the last frame's outputs to DIR/<name>.npy")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3

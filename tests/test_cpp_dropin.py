@@ -23,11 +23,13 @@ def test_core_api_example_compiles(tmp_path):
 
 
 def test_core_api_example_compiles_with_reference_sophus(tmp_path):
-    """With the reference's vendored Sophus + Eigen on the include path the pose type is Sophus::SE3d, as in the reference."""
-    ref = "/root/reference/third-party"
-    if not os.path.isdir(os.path.join(ref, "Sophus")):
-        pytest.skip("reference tree not present (GPU box)")
-    subprocess.check_call(["/usr/bin/g++", "-std=c++17", "-fsyntax-only", "-DEIGEN_MAX_ALIGN_BYTES=0", f"-I{ref}/Sophus", f"-I{ref}/Eigen",
+    """With the reference's vendored Sophus + Eigen on the include path the pose type is Sophus::SE3d, as in the reference. The
+    reference tree is the one oracle/Makefile builds from (REF)."""
+    ref = subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "print-ref"], capture_output=True, text=True).stdout.strip()
+    third = os.path.join(ref, "third-party")
+    if not ref or not os.path.isdir(os.path.join(third, "Sophus")):
+        pytest.skip("reference tree not present")
+    subprocess.check_call(["/usr/bin/g++", "-std=c++17", "-fsyntax-only", "-DEIGEN_MAX_ALIGN_BYTES=0", f"-I{third}/Sophus", f"-I{third}/Eigen",
                            f"-I{ROOT}/include/efusion", f"-I{ROOT}/include", SRC])
 
 

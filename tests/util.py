@@ -57,6 +57,36 @@ def run_oracle(frames, K, n, **kw):
     return f
 
 
+def tracking_inputs(frames, K):
+    """The inputs of one tracking step after three frames of the CPU oracle: frame 3's filtered depth and colour, frame 2's
+    colour, the oracle's pose and fill-in model maps (vertex, normal, image)."""
+    from oracle import ef_oracle as eo
+
+    f = run_oracle(frames, K, 3)
+    return dict(filt=eo.bilateral(frames[3][1], 3.0), rgba=rgba_of(frames[3][0]), prev_rgba=rgba_of(frames[2][0]), T=f.pose,
+                vtx=f.buffer("fill_vertex"), nrm=f.buffer("fill_normal"), img=f.buffer("fill_image"))
+
+
+def pose_inputs(T):
+    """Rcurr, tcurr, Rprev^-1, tprev of one ICP step: the pose T moved by a small rotation and translation."""
+    R = T[:3, :3].astype(np.float32)
+    t = T[:3, 3].astype(np.float32)
+    dR = np.array([[1, -0.002, 0.001], [0.002, 1, -0.003], [-0.001, 0.003, 1]], np.float32)
+    return (R @ dR).astype(np.float32), t + np.array([0.004, -0.003, 0.005], np.float32), np.linalg.inv(R).astype(np.float32), t
+
+
+def digest(arrays):
+    """sha256 over the names, shapes, dtypes and bytes of a dict of arrays."""
+    import hashlib
+
+    h = hashlib.sha256()
+    for k in sorted(arrays):
+        a = np.ascontiguousarray(arrays[k])
+        h.update(f"{k}{a.shape}{a.dtype.str}".encode())
+        h.update(a.tobytes())
+    return h.hexdigest()
+
+
 def oracle_sensitivity(frames, K, **cfg):
     """How far the ORACLE moves from itself when one depth pixel of frame 1 is 1 mm deeper: the scale below which a
     trajectory difference says nothing about an implementation (tracking amplifies any rounding difference the same way).
